@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W        (N>1: launched under torch.distributed.run)
   python bench.py --impl reference ...                 (CPU arm: the fp64 oracle port on the host cores)
+  python bench.py ... --dump-outputs DIR               (also write the last timed step's outputs as DIR/<name>.npy)
 
 A "step" is one RexGymEnv.step for every environment of the batch (one kernel launch); the workload is
 BASELINE.json configs[1]: 4096 envs/GPU, walk-ik, flat terrain, fused ABA+IK+motor kernel, synthetic
@@ -11,14 +12,16 @@ uniform random actions, training wrappers (ClipAction/RangeNormalize/LimitDurati
 (pinned) action buffers in and obs/reward/done back out every step.  Envs shard across GPUs with no data
 path collective (weak scaling).
 
-How the K steps are timed (round-1 verdict item 3: a 3 ms window measured scheduling noise, not the kernel):
-  * a BLOCK is exactly K steps, each bracketed by its own pair of CUDA events on the launching stream with the L2 flush
-    (256 MiB memset) between steps outside the events; the block's time is the sum of its K event intervals;
+How the K = --steps steps are timed (exactly K steps per workload; pick K large enough for the window you want):
+  * the K steps are split into BLOCKS of at most 200 consecutive steps; every step is bracketed by its own pair of CUDA events
+    on the launching stream with the L2 flush (256 MiB memset) between steps outside the events; a block's time is the sum of
+    its event intervals;
   * before a block the stream is parked behind a device-side gate (a spin kernel a few ms long) so the host enqueues the
     whole block ahead of the GPU: no host hiccup can land between an event and its kernel;
-  * the block is repeated until >= 100 ms of kernel time has been measured (at least 5 blocks); per block the MAX over ranks
-    is taken (barrier + synchronize on both sides of every block), and the MEDIAN block is reported: `ms_per_step` =
-    median block / K, `value` = envs x K / median block.  `timing` lists every block and every rank's own median;
+  * per block the MAX over ranks is taken (barrier + synchronize on both sides of every block); `ms_per_step` = the sum over
+    blocks / K, `value` = envs / ms_per_step.  The mean over the whole window, not a median over blocks: the step's cost
+    follows the gait phase of the batch, so blocks at different points of the window differ systematically, not by noise.
+    `timing` lists every block and every rank's own time per step;
   * the clocks come from ONE `nvidia-smi -lms 200` process per rank started before and stopped after the timed region
     (the profiling recipe's form), not from a process spawned every 200 ms.
 """
@@ -40,7 +43,7 @@ WORKLOAD = dict(task="walk", signal_type="ik", terrain_type="plane", target_posi
                 normalize=True, max_episode_steps=2000, auto_reset=True)
 # wall seconds per simulated second of the reference's own README recording (tests/test_readme_gif_clock.py: >= 3.6)
 DEMO_CLOCK = 4.0
-MIN_WINDOW_MS = 100.0
+BLOCK_STEPS = 200
 
 
 def b_alg(num_motors, A, O):
@@ -86,6 +89,12 @@ class ClockSampler(object):
                 "samples": len(rows)}
 
 
+def split_blocks(K):
+    """Sizes of the blocks K timed steps are split into: as even as possible, at most BLOCK_STEPS each, summing to K."""
+    nb = -(-K // BLOCK_STEPS)
+    return [K // nb + (1 if b < K % nb else 0) for b in range(nb)]
+
+
 def stagger_episodes(env, acts, span=256, groups=32):
     """Untimed: spread the episode ages of the batch uniformly over `span` control steps (reset 1/groups of the envs, step
     span/groups times, repeat).  After a common reset every env is in the same phase of the gait ramp and the step kernel's
@@ -105,12 +114,14 @@ def stagger_episodes(env, acts, span=256, groups=32):
 
 
 class Timer(object):
-    """Device-timed blocks of exactly K steps (see the module docstring)."""
+    """Device-timed blocks of consecutive steps (see the module docstring).  `last` holds what env.step returned in the
+    most recent timed step."""
 
     def __init__(self, dev, world, flush):
         import torch
         self.torch, self.dev, self.world, self.flush = torch, dev, world, flush
         self.clock_hz = 1.9e9
+        self.last = None
 
     def barrier(self):
         if self.world > 1:
@@ -126,49 +137,41 @@ class Timer(object):
         for k in range(K):
             self.flush.zero_()                                          # L2 flush between timed iterations (not timed)
             ev[k][0].record()
-            _, _, d, _ = env.step(acts[(first + k) % acts.shape[0]])
+            self.last = env.step(acts[(first + k) % acts.shape[0]])
             if after_step is not None:
                 after_step(env)
             ev[k][1].record()
             if done_acc is not None:
-                done_acc.add_(d.sum())
+                done_acc.add_(self.last[2].sum())
         self.barrier()
         return sum(a.elapsed_time(b) for a, b in ev)
 
-    def run(self, env, acts, first, K, after_step=None, min_window_ms=MIN_WINDOW_MS, min_blocks=5, max_blocks=400):
-        """-> dict(ms_per_step, block_ms [max over ranks per block], per_rank_ms_per_step, resets_per_step, launches)."""
+    def run(self, env, acts, first, K, after_step=None):
+        """Exactly K timed steps -> dict(ms_per_step, block_ms [max over ranks per block], per_rank_ms_per_step,
+        resets_per_step, launches)."""
         torch = self.torch
         done_acc = torch.zeros((), dtype=torch.int64, device=self.dev)
         l0 = env.launch_count
-        mine, blocks = [], 0
-        while True:
-            mine.append(self.block(env, acts, first + blocks * K, K, after_step, done_acc))
-            blocks += 1
-            t = torch.tensor([sum(mine), float(blocks)], dtype=torch.float64, device=self.dev)
-            if self.world > 1:
-                import torch.distributed as dist
-                dist.all_reduce(t, op=dist.ReduceOp.MIN)               # every rank stops at the same block count
-            if (blocks >= min_blocks and float(t[0]) >= min_window_ms) or blocks >= max_blocks:
-                break
+        sizes, mine = split_blocks(K), []
+        for kb in sizes:
+            mine.append(self.block(env, acts, first + sum(sizes[:len(mine)]), kb, after_step, done_acc))
         launches = env.launch_count - l0
         mine_t = torch.tensor(mine, dtype=torch.float64, device=self.dev)
         per_block = mine_t.clone()
-        per_rank = [float(mine_t.median())]
+        per_rank = [float(mine_t.sum()) / K]
         if self.world > 1:
             import torch.distributed as dist
             dist.all_reduce(per_block, op=dist.ReduceOp.MAX)
             g = [torch.zeros_like(mine_t) for _ in range(self.world)]
             dist.all_gather(g, mine_t)
-            per_rank = [float(x.median()) for x in g]
-        block_ms = sorted(float(x) for x in per_block)
-        med = block_ms[len(block_ms) // 2] if len(block_ms) % 2 else 0.5 * (block_ms[len(block_ms) // 2 - 1] + block_ms[len(block_ms) // 2])
+            per_rank = [float(x.sum()) / K for x in g]
         dn = done_acc.to(torch.float64)
         if self.world > 1:
             import torch.distributed as dist
             dist.all_reduce(dn)
-        return {"ms_per_step": med / K, "block_ms": [round(float(x), 5) for x in per_block], "blocks": blocks,
-                "window_ms": round(float(per_block.sum()), 3), "per_rank_ms_per_step": [round(x / K, 6) for x in per_rank],
-                "resets_per_step": float(dn) / (self.world * env.num_envs * K * blocks), "launches": int(launches), "steps_timed": K * blocks}
+        return {"ms_per_step": float(per_block.sum()) / K, "block_ms": [round(float(x), 5) for x in per_block], "block_steps": sizes, "blocks": len(sizes),
+                "window_ms": round(float(per_block.sum()), 3), "per_rank_ms_per_step": [round(x, 6) for x in per_rank],
+                "resets_per_step": float(dn) / (self.world * env.num_envs * K), "launches": int(launches), "steps_timed": K}
 
 
 def run_reference(args):
@@ -202,10 +205,12 @@ def run_reference(args):
             sim.reset(np.nonzero(d)[0])
     t0 = time.perf_counter()
     for k in range(args.warmup, args.warmup + args.steps):
-        _, _, d = sim.step(acts[k], nthreads=cores)
+        o, r, d = sim.step(acts[k], nthreads=cores)
         if d.any():
             sim.reset(np.nonzero(d)[0])
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"observ": o, "reward": r, "done": d})
     v = n * args.steps / dt
     cb = {"value": v, "unit": "env-steps/s", "cores": cores, "kind": "port",
           "sample": f"{n} envs x {args.steps} steps of the walk-ik flat workload, OpenMP over envs; NOT PyBullet (not installable "
@@ -245,6 +250,13 @@ def kernel_counts():
         return {}
 
 
+def dump_outputs(out_dir, arrays, rank=None):
+    """Write the last timed step's outputs as float32 DIR/<name>.npy (DIR/<name>_rank<r>.npy when sharded over ranks)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ("" if rank is None else "_rank%d" % rank) + ".npy"), np.asarray(a, np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -253,7 +265,11 @@ def main():
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--envs-per-gpu", type=int, default=ENVS_PER_GPU)
     ap.add_argument("--no-extras", action="store_true", help="headline + e2e only (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after timing, write what the last timed step returned (observ, reward, done, motor command) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -287,7 +303,7 @@ def main():
     except Exception:
         gpu_id = str(local)
 
-    def measure(kw, nb, Kb, min_window_ms, after_step=None, n_act=None):
+    def measure(kw, nb, Kb, after_step=None, n_act=None):
         """Create, de-synchronise, warm up and time one workload; returns the Timer dict + error flags."""
         env = R.BatchedRexEnv(num_envs=nb, device=f"cuda:{local}", seed=1234, env_offset=rank * nb, **kw)
         env.reset()
@@ -295,51 +311,51 @@ def main():
         stagger_episodes(env, acts)
         for k in range(W):
             env.step(acts[k % acts.shape[0]])
-        r = T.run(env, acts, W, Kb, after_step=after_step, min_window_ms=min_window_ms)
+        r = T.run(env, acts, W, Kb, after_step=after_step)
         r["error_flags_or"] = env.check_errors()
         r["envs_per_gpu"], r["value"], r["unit"] = nb, world * nb * 1e3 / r["ms_per_step"], "env-steps/s"
         return env, acts, r
 
     # ---- device-timed headline --------------------------------------------------------------------------------------
     sampler = ClockSampler(gpu_id)
-    env, acts, head = measure(WORKLOAD, n, K, MIN_WINDOW_MS, n_act=max(32, min(W + K, 256)))
+    env, acts, head = measure(WORKLOAD, n, K, n_act=max(32, min(W + K, 256)))
     A, O = env.action_dim, env.obs_dim
     value, ms_per_step = head["value"], head["ms_per_step"]
-    launches_per_block = head["launches"] / head["blocks"]
+    if args.dump_outputs:                   # what BatchedRexEnv.step handed its caller; info[i]["action"] = motor command row i
+        obs, reward, done, _ = T.last
+        dump_outputs(args.dump_outputs, {"observ": obs.cpu().numpy(), "reward": reward.cpu().numpy(), "done": done.cpu().numpy(),
+                                         "motor_command": env.last_command().t().cpu().numpy()}, rank if world > 1 else None)
 
-    # ---- end-to-end arm: host buffers through the public API, copies inside the timed region (blocks of K steps, wall clock) ----
+    # ---- end-to-end arm: host buffers through the public API, copies inside the timed region (the same K steps in the
+    # same blocks, wall clock) ----
     acts_h = acts.cpu().numpy()
     for k in range(3):
         env.step(acts_h[k])
-    e2e_blocks = []
-    while True:
+    e2e_blocks, k = [], 0
+    for kb in split_blocks(K):
         T.barrier()
         t0 = time.perf_counter()
-        for k in range(K):
+        for _ in range(kb):
             o, r, d, _ = env.step(acts_h[(W + k) % acts_h.shape[0]])
+            k += 1
         T.barrier()
         tl = torch.tensor([time.perf_counter() - t0], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(tl, op=dist.ReduceOp.MAX)
         e2e_blocks.append(float(tl.item()))
-        if (len(e2e_blocks) >= 5 and sum(e2e_blocks) >= MIN_WINDOW_MS * 1e-3) or len(e2e_blocks) >= 400:
-            break
-    e2e_s = sorted(e2e_blocks)[len(e2e_blocks) // 2]
-    e2e_value = world * n * K / e2e_s
+    e2e_value = world * n * K / sum(e2e_blocks)
     clocks = sampler.stop()
     err = env.check_errors()
     env.close()
 
     extras = {}
     if not args.no_extras:
-        Kb = min(K, 50)
-
         def extra(name, kw, nb, after_step=None, note=None):
             try:
-                e, _, r = measure(kw, nb, Kb, 50.0, after_step=after_step)
+                e, _, r = measure(kw, nb, K, after_step=after_step)
                 e.close()
                 keep = {k: r[k] for k in ("envs_per_gpu", "ms_per_step", "value", "unit", "resets_per_step", "error_flags_or", "blocks", "window_ms")}
-                keep["global_envs"], keep["steps"] = world * nb, Kb
+                keep["global_envs"], keep["steps"] = world * nb, K
                 if note:
                     keep["note"] = note
                 extras[name] = keep
@@ -438,13 +454,14 @@ def main():
                                       "simulation clock this model's forward trot tips over after ~240 control steps (1/240 = 0.0042); at the clock "
                                       "the reference's README recording ran at (x4, extras) it walks to the goal",
                        "error_flags_or": err, "extras": extras},
-            "timing": {"block_steps": K, "blocks": head["blocks"], "window_ms": head["window_ms"], "block_ms": head["block_ms"],
-                       "per_rank_ms_per_step": head["per_rank_ms_per_step"], "statistic": "median over blocks of the max over ranks",
+            "timing": {"steps_timed": head["steps_timed"], "block_steps": head["block_steps"], "blocks": head["blocks"],
+                       "window_ms": head["window_ms"], "block_ms": head["block_ms"], "per_rank_ms_per_step": head["per_rank_ms_per_step"],
+                       "statistic": "sum over blocks of the max over ranks, / steps_timed",
                        "e2e_blocks": len(e2e_blocks), "e2e_window_ms": round(1e3 * sum(e2e_blocks), 3)},
             "clocks": clocks,
             "e2e": {"value": e2e_value, "unit": "env-steps/s", "h2d_bytes_per_step": n * A * 4,
                     "d2h_bytes_per_step": n * (O * 4 + 4 + 1) + 4},
-            "gpu_launches": int(round(launches_per_block)),
+            "gpu_launches": head["launches"],
             "roofline": roof,
         }
         try:

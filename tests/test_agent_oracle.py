@@ -1,5 +1,6 @@
 """CPU: the numpy restatement of the agent glue (oracle/agent_oracle.py) against independent definitions, the TF-checkpoint
-reader against every policy the reference ships, and the C ABI of include/rexsim_agent.h (symbols only; no GPU here)."""
+reader against every policy the reference ships (tests/golden/policies: the shipped checkpoints cut to the variables the project
+restores, tools/gen_policy_golden.py), and the C ABI of include/rexsim_agent.h (symbols only; no GPU here)."""
 import os
 import re
 
@@ -9,7 +10,7 @@ import pytest
 from oracle import agent_oracle as AO
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_POLICIES = "/root/reference/rex_gym/policies"
+REF_POLICIES = os.path.join(ROOT, "tests", "golden", "policies")
 
 
 def test_agent_abi_exports_every_declared_symbol():
@@ -104,7 +105,6 @@ def test_noise_generator_is_the_kernels_generator():
     assert abs(z.mean()) < 0.06 and abs(z.std() - 1) < 0.05
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_POLICIES), reason="reference tree not present")
 def test_every_shipped_policy_loads():
     """rex_gym/policies/<task>/<signal>: TF checkpoint-V2 -> ForwardGaussianPolicy layout (200-100 layers, filters)."""
     from rex_gym_b200.agents import tf_checkpoint as tfc

@@ -10,7 +10,7 @@ import torch
 from oracle import agent_oracle as AO
 
 pytestmark = pytest.mark.gpu
-REF_POLICIES = "/root/reference/rex_gym/policies"
+REF_POLICIES = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "policies")
 
 
 def _random_weights(rng, O, A, H1=200, H2=100):
@@ -186,7 +186,6 @@ def test_rollout_graph_equals_the_step_by_step_loop():
     assert np.abs((a0["action"] - a0["mean"]).cpu().numpy()).max() > 1e-3   # training: sampled actions
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_POLICIES), reason="reference tree not present (never is on the GPU box)")
 def test_shipped_policy_runs_on_the_device():
     from rex_gym_b200.agents import ForwardGaussianPolicy
     net = ForwardGaussianPolicy.from_tf_checkpoint(os.path.join(REF_POLICIES, "gallop", "ol"))

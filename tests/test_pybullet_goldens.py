@@ -363,17 +363,20 @@ def test_recorded_trajectories_select_the_link_damping_and_the_toe_reach():
 
 
 def test_fixture_matches_the_reference_checkpoints():
-    """Regenerate-and-compare when the reference tree is present (it is not on the GPU box)."""
-    ref = "/root/reference/rex_gym/policies"
-    if not os.path.isdir(ref):
-        pytest.skip("reference tree not present")
-    from rex_gym_b200.agents import tf_checkpoint as tfc
+    """The fixture is the checkpoints' EpisodeMemory: compared with the rows of the same memory variables that
+    tests/golden/tf_memory_golden.npz samples from the first 400 steps of the same checkpoints (tools/gen_policy_golden.py)."""
+    M = np.load(os.path.join(os.path.dirname(__file__), "golden", "tf_memory_golden.npz"))
     for task in ("gallop", "walk", "turn", "standup"):
-        v = tfc.load_variables(tfc.latest_checkpoint(os.path.join(ref, task, "ol")), ["memory/Variable_1", "memory/Variable_2", "memory/Variable_5"])
-        n = G[task + "_ol_action"].shape[1]
-        np.testing.assert_array_equal(G[task + "_ol_observ"], v["memory/Variable_1"][:25, :n + 1])
-        np.testing.assert_array_equal(G[task + "_ol_action"], v["memory/Variable_2"][:25, :n])
-        np.testing.assert_array_equal(G[task + "_ol_reward"], v["memory/Variable_5"][:25, :n])
+        name = task + "_ol"
+        n = G[name + "_action"].shape[1]
+        ep, t = np.divmod(M[name + "_rows"], 400)
+        assert G[name + "_observ"].shape[0] == 25 and ep.max() == 24
+        k = t <= n
+        np.testing.assert_array_equal(G[name + "_observ"][ep[k], t[k]], M[name + "_observ"][k])
+        k = t < n
+        assert k.sum() >= 400, (task, k.sum())
+        np.testing.assert_array_equal(G[name + "_action"][ep[k], t[k]], M[name + "_action"][k])
+        np.testing.assert_array_equal(G[name + "_reward"][ep[k], t[k]], M[name + "_reward"][k])
 
 
 def _ripple_period(x, lo=5):
@@ -480,7 +483,6 @@ def test_wall_clock_gait_of_the_recorded_gallop_ik_episodes():
         assert abs(out[100:, 1].mean() - ref[ep, 101:401, 1].mean()) < 0.03      # mean pitch of the hopping gait
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/rex_gym/policies"), reason="needs the shipped TF checkpoint (reference tree)")
 def test_shipped_gallop_policy_closes_the_loop_like_its_training_runs():
     """End to end: the gallop-ol policy the reference ships (TF checkpoint -> pure-Python reader -> numpy restatement of
     ForwardGaussianPolicy + StreamingNormalize) drives the restated simulator.  It gallops forward (-x) for the whole
@@ -489,7 +491,7 @@ def test_shipped_gallop_policy_closes_the_loop_like_its_training_runs():
     a target x_ours(t) / reward(t), which has to fall in that range if the two simulators cover ground at the same rate."""
     from oracle import agent_oracle as AO
     from rex_gym_b200.agents.networks import read_tf_policy
-    w, filt = read_tf_policy("/root/reference/rex_gym/policies/gallop/ol")
+    w, filt = read_tf_policy(os.path.join(os.path.dirname(__file__), "golden", "policies", "gallop", "ol"))
     f = AO.StreamingNormalize((16,), True, True, 5)
     f.count, f.mean, f.var_sum = filt[0], np.array(filt[1], np.float64), np.array(filt[2], np.float64)
     s = OracleSim(1, "gallop", "ol", normalize=True, settle=2, target_position=2.0)
@@ -507,7 +509,6 @@ def test_shipped_gallop_policy_closes_the_loop_like_its_training_runs():
     assert np.sum((implied > 0.85) & (implied < 3.5)) >= 21, implied
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/rex_gym/policies"), reason="needs the shipped TF checkpoint (reference tree)")
 def test_shipped_walk_policy_reproduces_the_recorded_reward_profile():
     """The shipped walk-ol policy in closed loop on the restated simulator, target 2.0 m: ramps up, walks to the goal, brakes
     and stands still -- the per-step reward (rex_gym_env.py:501-542) has the profile of the 25 episodes PyBullet recorded in
@@ -515,7 +516,7 @@ def test_shipped_walk_policy_reproduces_the_recorded_reward_profile():
     0.3-0.4 m to stop past the goal: `tp - cx` once cx > tp + 0.15), and standing still for the rest of the 2000 steps."""
     from oracle import agent_oracle as AO
     from rex_gym_b200.agents.networks import read_tf_policy
-    w, filt = read_tf_policy("/root/reference/rex_gym/policies/walk/ol")
+    w, filt = read_tf_policy(os.path.join(os.path.dirname(__file__), "golden", "policies", "walk", "ol"))
     f = AO.StreamingNormalize((4,), True, True, 5)
     f.count, f.mean, f.var_sum = filt[0], np.array(filt[1], np.float64), np.array(filt[2], np.float64)
     s = OracleSim(1, "walk", "ol", normalize=True, settle=2, target_position=2.0, backwards=False)

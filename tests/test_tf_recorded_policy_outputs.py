@@ -8,28 +8,32 @@ enough to tell the architecture apart: the numpy restatement of StreamingNormali
 (oracle/agent_oracle.py, which tests/test_gpu_agent.py holds the CUDA kernel to) reproduces them to an rms of 0.02-0.08 (the
 policy's own stddev is 0.39), while dropping the mean layer's tanh, using tanh hidden units, not centring the observation or
 leaving the 1e-4 out of the variance are 2-25x worse.  The stored actions confirm the sampling law: (action - mean) / exp(logstd)
-is a unit normal."""
+is a unit normal.
+
+The checkpoints and the recorded memory are golden fixtures (tools/gen_policy_golden.py): tests/golden/policies holds the shipped
+checkpoints cut to the networks and normalisers, tests/golden/tf_memory_golden.npz a seeded sample of 1200 of the 25 x 400
+recorded (observation, mean) rows for the forward pass, and the log-stddevs and the sampling noise (action - mean, half precision) of
+all 25 x 400 rows for the sampling law."""
 import os
 
 import numpy as np
 import pytest
 
-ROOT = "/root/reference/rex_gym/policies"
-pytestmark = pytest.mark.skipif(not os.path.isdir(ROOT), reason="needs the shipped TF checkpoints (reference tree)")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+ROOT = os.path.join(GOLDEN, "policies")
+MEMORY = np.load(os.path.join(GOLDEN, "tf_memory_golden.npz"))
 CKPTS = [("gallop", "ik"), ("gallop", "ol"), ("standup", "ol"), ("turn", "ik"), ("turn", "ol"), ("walk", "ik"), ("walk", "ol")]
 
 
-def _load(task, sig, steps=400):
+def _load(task, sig):
+    """Sampled rows: observation and recorded mean; whole 25 x 400 window: recorded log-stddev and action - mean."""
     from oracle import agent_oracle as AO
-    from rex_gym_b200.agents import tf_checkpoint as tfc
     from rex_gym_b200.agents.networks import read_tf_policy
-    p = os.path.join(ROOT, task, sig)
-    v = tfc.load_variables(tfc.latest_checkpoint(p), ["memory/Variable_1", "memory/Variable_2", "memory/Variable_3", "memory/Variable_4"])
-    w, filt = read_tf_policy(p)
-    obs, act, mean, logstd = (v["memory/Variable_%d" % k][:, :steps] for k in (1, 2, 3, 4))
+    w, filt = read_tf_policy(os.path.join(ROOT, task, sig))
+    obs, mean, logstd, noise = (MEMORY["%s_%s_%s" % (task, sig, k)] for k in ("observ", "mean", "logstd", "noise"))
     f = AO.StreamingNormalize((obs.shape[-1],), True, True, 5)
     f.count, f.mean, f.var_sum = filt[0], np.array(filt[1], np.float64), np.array(filt[2], np.float64)
-    return AO, w, f, obs.astype(np.float64), act, mean, logstd
+    return AO, w, f, obs.astype(np.float64), mean, logstd, noise.astype(np.float64)
 
 
 def _variant(w, f, x, variant):
@@ -48,8 +52,7 @@ def _variant(w, f, x, variant):
 
 @pytest.mark.parametrize("task,sig", CKPTS)
 def test_forward_pass_reproduces_the_means_tensorflow_recorded(task, sig):
-    AO, w, f, obs, act, mean, logstd = _load(task, sig)
-    x = obs.reshape(-1, obs.shape[-1])
+    AO, w, f, x, mean, logstd, noise = _load(task, sig)
     _, m, _, _ = AO.perform(w, f, x, False)
     m = np.asarray(m).reshape(mean.shape)
     rms = float(np.sqrt(((m - mean) ** 2).mean()))
@@ -60,7 +63,7 @@ def test_forward_pass_reproduces_the_means_tensorflow_recorded(task, sig):
     # update that happened while these episodes were being collected (the 25 agents run in parallel, an update lands in the
     # middle of the others' episodes) -- all within 2e-2 of the saved one
     assert len(np.unique(logstd[..., 0])) <= 6 and np.abs(logstd - w["logstd"]).max() < 2e-2
-    z = (act - mean) / np.exp(logstd)                            # action = mean + exp(logstd) * N(0, 1)  (algorithm.py:117-121)
+    z = noise / np.exp(logstd)                                   # action = mean + exp(logstd) * N(0, 1)  (algorithm.py:117-121)
     assert abs(z.mean()) < 0.02 and 0.97 < z.std() < 1.03 and abs((np.abs(z) < 1).mean() - 0.6827) < 0.01
 
 
@@ -70,8 +73,7 @@ def test_forward_pass_reproduces_the_means_tensorflow_recorded(task, sig):
     ("gallop", "ol", "no_centre", 8.0), ("standup", "ol", "no_centre", 4.0), ("walk", "ik", "no_centre", 2.0),
     ("gallop", "ol", "no_variance_epsilon", 4.0), ("walk", "ik", "no_variance_epsilon", 8.0), ("turn", "ol", "no_variance_epsilon", 4.0)])
 def test_recorded_means_tell_the_architecture_apart(task, sig, variant, factor):
-    AO, w, f, obs, act, mean, logstd = _load(task, sig)
-    x = obs.reshape(-1, obs.shape[-1])
+    AO, w, f, x, mean, logstd, noise = _load(task, sig)
     rms = lambda m: float(np.sqrt(((m.reshape(mean.shape) - mean) ** 2).mean()))
     ours, other = rms(_variant(w, f, x, "ours")), rms(_variant(w, f, x, variant))
     _, ref, _, _ = AO.perform(w, f, x, False)
